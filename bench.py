@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — GC-ADPCM batch encode throughput on B200 (BASELINE.json metric), one JSON line on rank 0.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--channels C] [--seconds S]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--channels C] [--seconds S] [--dump-outputs DIR]
 
 A "step" = one pass of the hot path (coefficient analysis + exhaustive encode, GcAdpcmFormat.EncodeFromPcm16's loop)
 over one synthetic batch.  Default workload = BASELINE.json configs[1]: 1024 channels x 30 s x 48 kHz PCM16 per GPU
@@ -15,6 +15,9 @@ over one synthetic batch.  Default workload = BASELINE.json configs[1]: 1024 cha
   cpu_baseline  the CPU oracle port of the reference (oracle/, C, one task per channel on all host cores) on a bounded
              sample of the same batch.
 --impl reference times that CPU port alone (the reference itself is C#/.NET and cannot run in this image).
+--dump-outputs DIR  after the timed steps, writes what the last step computed as DIR/coefs.npy and DIR/adpcm.npy (float32,
+             one row per channel; a fixed seeded sample of the channels when all of them would exceed 64 MB).  The
+             inputs are seeded, so two builds run with the same arguments can be compared output for output.
 """
 from __future__ import annotations
 
@@ -57,11 +60,36 @@ def parse_args():
     ap.add_argument("--out-format", default="dsp", choices=["dsp", "adx", "hca"], help="batch: container to write")
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-cpu", action="store_true")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", help="c2 / --impl reference: write the last timed step's coefficients "
+                    "and ADPCM bytes as float32 .npy files under DIR")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "ours" and args.config != "c2":
+        ap.error("--dump-outputs is implemented for --config c2")
+    return args
 
 
 def env_rank():
     return int(os.environ.get("RANK", "0")), int(os.environ.get("LOCAL_RANK", "0")), int(os.environ.get("WORLD_SIZE", "1"))
+
+
+DUMP_BYTES = 60 * 1000 * 1000  # array data of --dump-outputs: with the .npy headers, under 64 MB
+
+
+def dump_sample(n_ch: int, n_bytes: int):
+    """(channels, ADPCM width) that --dump-outputs writes: every channel when all of them fit DUMP_BYTES as float32, else a
+    fixed seeded sample of whole channels (or the leading ADPCM bytes of one channel, if one alone does not fit)."""
+    k = max(1, min(n_ch, DUMP_BYTES // (4 * (16 + n_bytes))))
+    width = min(n_bytes, DUMP_BYTES // (4 * k) - 16)
+    rows = np.arange(n_ch) if k == n_ch else np.sort(np.random.default_rng(0x5647).choice(n_ch, k, replace=False))
+    return rows, width
+
+
+def dump_outputs(out_dir: str, **arrays):
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), np.asarray(a, dtype=np.float32))
 
 
 # ------------------------------------------------------------------------------------------------------------
@@ -215,9 +243,12 @@ def main():
         used = 1
         for i in range(args.warmup + args.steps):
             t0 = time.perf_counter()
-            _, _, used = pyoracle.encode_batch(pcm, 0)
+            coefs, adpcm, used = pyoracle.encode_batch(pcm, 0)
             if i >= args.warmup:
                 times.append(time.perf_counter() - t0)
+        if args.dump_outputs:
+            rows, width = dump_sample(*adpcm.shape)
+            dump_outputs(args.dump_outputs, coefs=coefs[rows], adpcm=adpcm[rows, :width])
         ms = 1e3 * sum(times) / len(times)
         value = sample_ch * n / (ms / 1e3) / 1e6
         line = {
@@ -324,6 +355,10 @@ def main():
         dist.all_reduce(tmax, op=dist.ReduceOp.MAX)
         elapsed_ms = float(tmax.item())
     barrier()
+    if args.dump_outputs and rank == 0:
+        rows, width = dump_sample(n_ch, n_bytes)
+        idx = torch.from_numpy(rows).to(device)
+        dump_outputs(args.dump_outputs, coefs=coefs_dev[idx].cpu().numpy(), adpcm=adpcm_dev[idx, :width].cpu().numpy())
     kernel_ms /= args.steps
     ms_per_step = elapsed_ms / args.steps
     value = world * samples_per_step / (ms_per_step / 1e3) / 1e6
@@ -345,7 +380,7 @@ def main():
             N.check(vg.lib.vgb_gcadpcm_encode_batch(in_tab, lens.ctypes.data, None, None, n_ch, coefs_host.ctypes.data,
                                                     out_tab, None, None))
 
-        e2e_steps = max(1, min(args.steps, 3))
+        e2e_steps = args.steps
         step_e2e()  # warm-up (allocates the library's own device buffers)
         barrier()
         t0 = time.perf_counter()
